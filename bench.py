@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """bench.py — frames/s of the PoseCNN hot path on synthetic 640x480 batches (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload full|hough|rgbd|project] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload full|hough|rgbd|project|train] [--batch B]
+                    [--dump-outputs DIR]
     python bench.py --impl reference ...      # the same path restated on the host cores (oracle/cpu_pipeline.py)
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over ONE GLOBAL batch of `--batch` synthetic
@@ -155,6 +156,45 @@ def profile_json(name):
         return None
 
 
+DUMP_BYTES = 60 * 1000 * 1000     # array data of --dump-outputs; with the .npy headers it stays under 64 MB
+_OUTPUTS = None     # host copies of what the timed path returned in its last step (--dump-outputs)
+
+
+def keep_outputs(named):
+    """Copy the tensors of `named` (nested dicts flattened as `outer.inner`) to the host for --dump-outputs: float64 stays
+    float64, everything else becomes float32.  Each array gets an equal share of DUMP_BYTES; a larger one is replaced
+    by its elements at a fixed sample of flat indices (numpy default_rng(0).choice(numel, share, replace=False), sorted),
+    so that two runs or two builds sample the same elements."""
+    import torch
+    flat = {}
+
+    def walk(d, pre):
+        for k, v in d.items():
+            if isinstance(v, dict):
+                walk(v, pre + k + ".")
+            elif torch.is_tensor(v):
+                flat[(pre + k).replace("/", "_")] = v.detach()
+    walk(named, "")
+    share = DUMP_BYTES // max(1, len(flat))
+    global _OUTPUTS
+    _OUTPUTS = {}
+    for name, t in flat.items():
+        dt = torch.float64 if t.dtype == torch.float64 else torch.float32
+        k = share // dt.itemsize
+        if t.numel() > k:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), k, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+            name += ".sample"
+        _OUTPUTS[name] = t.to(dt).cpu().numpy()
+    return _OUTPUTS
+
+
+def write_outputs(out_dir):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in _OUTPUTS.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------
 # Hough workload: batch of synthetic label / vertex maps (SURVEY §8(d) scenes; configs[1] scaled to batch B)
 # ------------------------------------------------------------------------------------------
@@ -178,7 +218,7 @@ def hough_inputs(batch, rank):
     return dict(label=tile(sc["label"]), vertex=tile(sc["vertex"]), meta=tile(sc["meta"]), extents=sc["extents"])
 
 
-def measure_hough(B, rank, world, local, steps, warmup, use_graph=True, e2e_batch=32, want_e2e=True):
+def measure_hough(B, rank, world, local, steps, warmup, use_graph=True, e2e_batch=32, want_e2e=True, dump=False):
     """Device time of the Houghvotinggpu op alone (dense vertex_pred input, the registered op signature) on the §8(d)
     scenes: CUDA-graph replay of the one C call (7 launches + 1 memset node), L2 flushed between timed iterations."""
     import torch
@@ -228,6 +268,8 @@ def measure_hough(B, rank, world, local, steps, warmup, use_graph=True, e2e_batc
         evs.append((e0, e1))
     torch.cuda.synchronize()
     barrier(world)
+    if dump:
+        keep_outputs(dict(zip(("rois", "poses", "poses_target", "poses_weight", "domain", "num_rois", "status"), out)))
     ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = max_over_ranks(float(np.sum(ms)), world)
     ms_step = total_ms / steps
@@ -260,7 +302,7 @@ def measure_hough(B, rank, world, local, steps, warmup, use_graph=True, e2e_batc
 
         e2e_step()
         torch.cuda.synchronize()
-        k = max(2, min(steps, 5))
+        k = steps
         t0 = time.perf_counter()
         for _ in range(k):
             e2e_step()
@@ -286,7 +328,8 @@ def run_hough(args, rank, world, local):
     B = args.batch
     sampler = ClockSampler(local)
     sampler.start()
-    rec = measure_hough(B, rank, world, local, args.steps, args.warmup, not args.no_graph, args.e2e_batch, not args.no_e2e)
+    rec = measure_hough(B, rank, world, local, args.steps, args.warmup, not args.no_graph, args.e2e_batch, not args.no_e2e,
+                        args.dump_outputs and rank == 0)
     clocks = sampler.stop()
     peaks = measured_peaks()
     traffic = profile_json("r02_hough_traffic.json")
@@ -328,7 +371,7 @@ def rotating_inputs(h_img_np, dev, min_bytes=140 * 1024 * 1024, max_bufs=48):
 
 
 def measure_pipeline(net, imgs_np, meta, ext, rank, world, dev, steps, warmup, batch_global, batch_offset, use_graph, want_e2e,
-                     extra_inputs=None):
+                     extra_inputs=None, dump=False):
     """K timed steps of the sharded pipeline: graph replay on the compute stream, records all-gathered on the
     communication stream (double-buffered), one event pair around the whole region, max over ranks."""
     import torch
@@ -371,6 +414,8 @@ def measure_pipeline(net, imgs_np, meta, ext, rank, world, dev, steps, warmup, b
     ms_step = max_over_ranks(e0.elapsed_time(e1) / steps, world)
     in_step_gather_ms = float(np.mean([pipe.last_gather_ms(last), pipe.last_gather_ms(last - 1)])) if steps >= 2 else None
     gathered = pipe.results(last)
+    if dump:    # before anything below runs the step again and overwrites the graph's output buffers
+        keep_outputs(dict(L, records_gathered=gathered))
     ndet = int((gathered[:, -1] > 0).sum().item())
     out = dict(ms_step=ms_step, layers=L, detections=ndet, nbufs=len(bufs), pipe=pipe, in_step_gather_ms=in_step_gather_ms, step=step,
                bufs=bufs)
@@ -410,7 +455,7 @@ def measure_pipeline(net, imgs_np, meta, ext, rank, world, dev, steps, warmup, b
 
         run_e2e(2)
         barrier(world)
-        k = max(steps, 30)       # the first upload cannot overlap anything: amortised over >= 30 steps like a serving loop's steady state
+        k = steps               # wall clock over the timed steps; the first upload of the window cannot overlap anything
         t0 = time.perf_counter()
         run_e2e(k)
         dt = max_over_ranks((time.perf_counter() - t0) / k, world)
@@ -450,7 +495,7 @@ def run_full(args, rank, world, local, input_format="COLOR"):
     sampler = ClockSampler(local)
     sampler.start()  # nvidia-smi needs ~100 ms to produce its first sample: start before the warm-up steps
     m = measure_pipeline(net, rgb_all[off:off + Bl], meta_all[off:off + Bl], ext, rank, world, dev, args.steps, args.warmup, Bg, off,
-                         not args.no_graph, not args.no_e2e, extra_shard)
+                         not args.no_graph, not args.no_e2e, extra_shard, args.dump_outputs and rank == 0)
     clocks = sampler.stop()
     ms_step, L, e2e = m["ms_step"], m["layers"], m.get("e2e")
     nlabels = int((L["label_2d"] > 0).sum().item())
@@ -491,7 +536,7 @@ def run_full(args, rank, world, local, input_format="COLOR"):
     flush = torch.empty(256 * 1024 * 1024, dtype=torch.uint8, device=dev)
     d_img = m["bufs"][0]
     tr = []
-    for _ in range(max(3, min(args.steps, 10))):
+    for _ in range(args.steps):
         flush.zero_()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); net._trunk(d_img); e1.record()
@@ -502,7 +547,7 @@ def run_full(args, rank, world, local, input_format="COLOR"):
     # Houghvotinggpu alone as the pipeline runs it (vertex head sampled from `lowres`) on the network's own label maps
     from posecnn_b200.hough_voting_gpu_layer import hough_voting_gpu_op as hop
     hs = []
-    for _ in range(5):
+    for _ in range(args.steps):
         flush.zero_()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
@@ -622,13 +667,15 @@ def run_project(args, rank, world, local):
     barrier(world)
     clocks = sampler.stop()
     ms_step = max_over_ranks(e0.elapsed_time(e1) / args.steps, world)
+    if args.dump_outputs and rank == 0:
+        keep_outputs(dict(project=out))
     # the dominant kernel alone
     tb0.record()
-    for _ in range(3):
+    for _ in range(args.steps):
         td = bop.backproject(data, lab, depth, meta, l3, G, ks, thr)
     tb1.record()
     torch.cuda.synchronize()
-    bp_ms = tb0.elapsed_time(tb1) / 3
+    bp_ms = tb0.elapsed_time(tb1) / args.steps
     peaks = measured_peaks()
     bp_bytes = Bl * G ** 3 * (2 * Cf + C) * 4 + Bl * H * W * (Cf + C + 1) * 4
     pj_bytes = Bl * H * W * (4 + 8 * Cf)
@@ -648,9 +695,9 @@ def run_project(args, rank, world, local):
 
         e2e_step()
         t0 = time.perf_counter()
-        for _ in range(3):
+        for _ in range(args.steps):
             e2e_step()
-        dt = max_over_ranks((time.perf_counter() - t0) / 3, world)
+        dt = max_over_ranks((time.perf_counter() - t0) / args.steps, world)
         e2e = dict(value=eb * world / dt, unit="frames/s", batch_per_gpu=eb, h2d_bytes_per_step=int((h_data.numel() + h_lab.numel() + h_depth.numel()) * 4),
                    d2h_bytes_per_step=int(h_out.numel() * 4), note="pinned host feature / label / depth maps in, projected features out")
     res = dict(
@@ -724,6 +771,8 @@ def run_train(args, rank, world, local):
     torch.cuda.synchronize(); barrier(world)
     clocks = sampler.stop()
     ms_step = max_over_ranks(e0.elapsed_time(e1) / args.steps, world)
+    if args.dump_outputs and rank == 0:
+        keep_outputs(out)
     # end to end: pinned host images + label maps in, the loss scalar out, every step; the upload of step i + 1 runs on a copy stream
     # while step i computes (double-buffered device inputs), as a training loop with a prefetching loader does
     d_in = [torch.empty_like(data) for _ in range(2)]
@@ -757,7 +806,7 @@ def run_train(args, rank, world, local):
 
     run_e2e(2)                                    # first touch of the staging buffers, allocator growth
     barrier(world)
-    k = max(6, args.steps)
+    k = args.steps
     t0 = time.perf_counter()
     run_e2e(k)
     dt = max_over_ranks((time.perf_counter() - t0) / k, world)
@@ -871,7 +920,7 @@ def main():
     claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every timed loop of the workload")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="full", choices=["hough", "full", "rgbd", "project", "train"])
@@ -883,7 +932,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling record of multi-GPU runs")
     ap.add_argument("--no-hough-record", action="store_true", help="skip the Hough-op sub-records of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path computed in its last timed step as DIR/<name>.npy "
+                                                          "(float32 / float64, sampled to at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     if args.impl == "reference":
         rank = int(os.environ.get("RANK", "0"))
@@ -910,7 +965,7 @@ def main():
             peaks = measured_peaks()
             hb = {}
             for B in (32, 1):
-                r = measure_hough(B, 0, 1, 0, max(args.steps, 10), args.warmup, True, 32, True)
+                r = measure_hough(B, 0, 1, 0, args.steps, args.warmup, True, 32, True)
                 r["frac"] = r["footprint_gbs"] / peaks["hbm_gbs"]
                 hb["b%d" % B] = r
             traffic = profile_json("r02_hough_traffic.json")
@@ -930,6 +985,8 @@ def main():
             res["roofline_hough"] = dict(bound="hbm", achieved=hb["b32"]["footprint_gbs"], peak=peaks["hbm_gbs"], unit="GB/s",
                                          frac=hb["b32"]["frac"], ms=hb["b32"]["device_ms"], scenes="SURVEY 8(d) synthetic scenes, batch 32")
     if rank == 0:
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs)
         if not args.no_cpu_baseline and world == 1 and args.workload in ("full",):
             try:
                 res["cpu_baseline"] = cpu_pipeline_sample(1, 4, 1)

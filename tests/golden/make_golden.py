@@ -39,6 +39,13 @@ def main(out_dir):
             d["votes"] = v.astype(np.int16)
         np.savez_compressed(os.path.join(out_dir, name + ".npz"), **d)
         print(name, "rows", nr, "max votes", v.max())
+    # the reference launcher as shipped (atomicAdd list order): with skip_pixels = 1 every pixel votes, so its rows
+    # are order independent as a set
+    sc, _, vt, pt, _ = cases.hough_inputs("h_skip1_d")
+    outs, nr = ref.hough_full(T(sc["label"]), T(sc["vertex"]), T(sc["extents"]), T(sc["meta"]), T(sc["gt"]), 0, vt, pt, 1)
+    np.savez_compressed(os.path.join(out_dir, "h_skip1_d_shipped.npz"), box=N(outs[0]), pose=N(outs[1]), target=N(outs[2]),
+                        weight=N(outs[3]), domain=N(outs[4]), num_rois=np.int32(nr))
+    print("h_skip1_d_shipped rows", nr)
     data, rois, grad = cases.roi_inputs()
     top, arg = ref.roi_pool(T(data), T(rois), 7, 7, 1.0 / 16.0, 0)
     gin = ref.roi_pool_grad(T(data), T(rois), arg, T(grad), 7, 7, 1.0 / 16.0, 0)

@@ -288,7 +288,7 @@ def test_bench_reference_arm_prints_one_json_line():
     assert d["impl"] == "reference" and d["value"] > 0 and d["cpu_baseline"]["cores"] >= 1 and d["e2e"]["value"] == d["value"]
 
 
-# lib/networks/network.py:6-26, verbatim (checked against the file where /root/reference is mounted)
+# lib/networks/network.py:6-26, verbatim
 NETWORK_PY_IMPORTS = """\
 import backprojecting_layer.backprojecting_op as backproject_op
 import backprojecting_layer.backprojecting_op_grad
@@ -312,6 +312,8 @@ import gradient_reversal_layer.gradient_reversal_op_grad
 import hard_label_layer.hard_label_op as hard_label_op
 import hard_label_layer.hard_label_op_grad
 """
+# sha256 of lines 6-26 of the reference's lib/networks/network.py (newline-terminated), taken from the file itself
+NETWORK_PY_IMPORTS_SHA256 = "c9cf9ad65096914c4b85d5c10480df5f85f7a3050d33cd36294d9d8b6a0bd79a"
 
 # the op symbols lib/networks/network.py calls on those modules (network.py:226-340)
 NETWORK_PY_SYMBOLS = {
@@ -329,12 +331,10 @@ def test_reference_import_paths_resolve():
     """Replays EVERY op import statement of lib/networks/network.py:6-26 verbatim with posecnn_b200/ on sys.path (the
     way the reference puts lib/ on it, tools/_init_paths.py): all 21 must resolve, every symbol network.py uses must be
     callable, and the out-of-scope ops (SURVEY.md §8(b) stubs) must fail loudly when called instead of falling back."""
+    import hashlib
     import subprocess
     import sys
-    ref = "/root/reference/lib/networks/network.py"
-    if os.path.exists(ref):
-        lines = open(ref).read().splitlines()[5:26]
-        assert "\n".join(lines) + "\n" == NETWORK_PY_IMPORTS
+    assert hashlib.sha256(NETWORK_PY_IMPORTS.encode()).hexdigest() == NETWORK_PY_IMPORTS_SHA256
     prog = (
         "import sys; sys.path.insert(0, %r); sys.path.insert(0, %r)\n" % (ROOT, os.path.join(ROOT, "posecnn_b200"))
         + NETWORK_PY_IMPORTS

@@ -1,4 +1,4 @@
-"""N = 2 over NCCL (needs two GPUs: `gpurun --gpus 2 -- python -m pytest tests/test_multigpu_nccl_gpu.py -m gpu`):
+"""N = 2 over NCCL (needs two GPUs: `python -m pytest tests/test_multigpu_nccl_gpu.py -m gpu` on a machine with two):
 the gathered post-NMS records of two image shards of ONE global batch equal the single-GPU records (SURVEY.md §8(e))."""
 import os
 import socket
@@ -49,7 +49,7 @@ print("RANK_OK", rank, whole.shape[0])
 
 def test_two_rank_gather_equals_single_gpu(tmp_path):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     script = tmp_path / "worker.py"
     script.write_text(WORKER)
@@ -111,7 +111,7 @@ def test_two_rank_training_step_equals_single_gpu(tmp_path):
     """configs[4] contract: one SGD step on image shards over 2 ranks (global loss normalisers, NCCL all-reduce of the gradients)
     == the step on the whole batch on one GPU (gradients to 2e-3 relative: only the fp32 summation order differs)."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     script = tmp_path / "train_worker.py"
     script.write_text(TRAIN_WORKER)
